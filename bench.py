@@ -7,8 +7,12 @@ One "step" = one full gradient evaluation of the ensemble: forward solve + fused
 reduction (+ the one all-reduce of dp over ranks for N>1, issued by b200adj_reverse itself through the handle's NCCL
 communicator; members are sharded, weak scaling: 65536 per GPU).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--members M]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--members M] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
+
+--dump-outputs DIR writes what the timed C2 loop hands its caller after its last step, DIR/dp.npy [3] and DIR/du0.npy [3, N]
+(rank 0's members), both float64.  The inputs are seeded, so two builds run with the same arguments can be compared array
+for array.  Above 60 MB du0 is thinned to every k-th member (the smallest k that fits).
 
 Keys of the one JSON line (rank 0):
 `value`     members/s with inputs resident in HBM (device pointers through the C ABI), CUDA-event timed, max over ranks.
@@ -26,6 +30,7 @@ Keys of the one JSON line (rank 0):
 `cpu_baseline` the C oracle (a PORT of the reference algorithm; Julia cannot run here) on the host cores.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -43,6 +48,7 @@ ALG_BYTES_PER_MEMBER_STEP = 8 * (3 + 2 * 6 + 101.0 / 1000.0 * 3)   # 122.4 B (SU
 # fp64 work of one reverse member-step (cuobjdump -sass of tsit5_reverse_kernel<Lorenz,GAUSS>, DESIGN.md 4.2)
 DP_INSTR_PER_MEMBER_STEP = dict(dfma=366, dmul=33, dadd=27)
 PARITY_TOL = 1e-8
+DUMP_BYTES = 60_000_000
 
 
 def make_inputs(N, offset=0):
@@ -145,6 +151,7 @@ class ClockSampler:
             self.f = open(self.path, "w")
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "20",
                                           "-i", str(self.device)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)          # a run that dies before stop() must not leave the sampler behind
         except Exception:
             self.proc = None
 
@@ -522,6 +529,8 @@ def run_ours(args):
     ms_per_step = total_ms / args.steps
     value = N * world / (ms_per_step * 1e-3)
     dp_check = main.dp.cpu().numpy().tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main.du0.cpu().numpy(), main.dp.cpu().numpy())
     main.close()
 
     # ---------------- end-to-end arms: public API, host buffers ----------------
@@ -801,6 +810,14 @@ def _quiet_stdout():
     os.dup2(2, 1)
 
 
+def dump_outputs(out_dir, du0, dp):
+    """dp whole; du0 [d, N] at the smallest member stride that keeps it within DUMP_BYTES"""
+    os.makedirs(out_dir, exist_ok=True)
+    stride = -(-du0.nbytes // DUMP_BYTES)
+    np.save(os.path.join(out_dir, "dp.npy"), dp)
+    np.save(os.path.join(out_dir, "du0.npy"), np.ascontiguousarray(du0[:, ::stride]))
+
+
 def emit(line):
     data = (json.dumps(line) + "\n").encode()
     if _REAL_STDOUT is None:
@@ -821,7 +838,12 @@ def main():
     ap.add_argument("--dtype", default="", help="c4 only: bf16_f32acc (default), f32 or f64")
     ap.add_argument("--no-secondary", action="store_true", help="skip the sharded C4 / C5 legs (profiling runs)")
     ap.add_argument("--nccl-allreduce", action="store_true", help="N > 1: ncclAllReduce instead of the fused peer-memory all-reduce (A/B)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write du0 and dp of the last timed C2 step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs applies to the C2 device run (--impl ours --workload c2)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     Shard.nccl_allreduce = args.nccl_allreduce

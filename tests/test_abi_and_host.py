@@ -215,6 +215,27 @@ def test_bench_secondary_specs_are_consistent_with_the_oracle():
         assert 0.0 < rf["frac"] < 10.0 and sp["cpu_sample"] >= sp["parity_members"]
 
 
+def test_bench_dump_outputs_stays_within_64_mb(tmp_path):
+    """bench.py --dump-outputs: dp whole, du0 whole while it fits, else every k-th member for the smallest k that fits; the
+    flag is refused where there is no C2 device run to dump, and --steps below 1 is refused."""
+    import importlib.util
+    import subprocess
+    import sys
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
+    dp = np.array([1.0, 2.0, 3.0])
+    du0 = np.arange(3 * 3_000_000, dtype=np.float64).reshape(3, -1)            # 72 MB
+    bench.dump_outputs(str(tmp_path), du0, dp)
+    assert np.array_equal(np.load(tmp_path / "dp.npy"), dp)
+    assert np.array_equal(np.load(tmp_path / "du0.npy"), du0[:, ::2])
+    assert sum(f.stat().st_size for f in tmp_path.iterdir()) <= 64e6
+    bench.dump_outputs(str(tmp_path), du0[:, :1000], dp)
+    assert np.array_equal(np.load(tmp_path / "du0.npy"), du0[:, :1000])
+    for extra in (["--impl", "reference", "--dump-outputs", str(tmp_path)], ["--workload", "c1", "--dump-outputs", str(tmp_path)], ["--steps", "0"]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert res.returncode == 2, (extra, res.stderr)
+
+
 def test_bench_reference_arm_contract():
     """`bench.py --impl reference` (the CPU arm the driver runs first): exactly one JSON line on stdout with the contract's
     keys, measured on the oracle port; other ranks of a torchrun launch print nothing and exit 0."""
